@@ -13,7 +13,7 @@ the on-device FIFO / MWR rules), each with its algorithmic bytes and HBM-rooflin
 "cpu_baseline" the reference's CPU path timed on this box's host cores: the C oracle port AND the
 unmodified Python reference (oracle/_ref, installed by oracle/install_ref.py).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs all|none]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs all|none] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -319,6 +319,24 @@ def config_entry(workload, n_total, ms, steps, mean_balg, peak, launches, world=
     return d
 
 
+def dump_outputs(directory, env, acts, torch, budget=60_000_000):
+    """Write what the last timed step_sample() returned to its caller as float32 .npy files (exact: every value is
+    float32 already or an integer below 2**24), so that two builds can be compared output for output.  When the batch
+    exceeds `budget` bytes, a fixed seeded sample of the envs is written; env_index.npy holds their indices."""
+    import numpy as np
+    arrays = {"real_obs": env.real_obs, "action_mask": env.action_mask, "reward": env.reward, "done": env.done,
+              "truncated": env._truncated, "next_actions": acts}
+    n = env.num_envs
+    row_bytes = 4 * (1 + sum(int(np.prod(a.shape[1:])) for a in arrays.values()))
+    rows = min(n, budget // row_bytes)
+    idx = np.arange(n) if rows == n else np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+    sel = torch.as_tensor(idx, device=env.device)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "env_index.npy"), idx.astype(np.float32))
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a.index_select(0, sel).float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -334,6 +352,7 @@ def main():
     ap.add_argument("--no-preroll", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     ap.add_argument("--py-ref-worker", nargs=3, metavar=("INSTANCE", "SECONDS", "SEED"), help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.py_ref_worker:
@@ -391,6 +410,8 @@ def main():
     elapsed_ms, launches, acts = time_fused_steps(env, "RANDOM", acts, W, K, torch, dist, world)
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env, acts, torch)
     # the timed region is K launches of ONE kernel (the fused step), bracketed by CUDA events on the
     # launching stream: its average launch duration is elapsed / K (launch gaps, if any, count against us)
     step_kernel_ms = elapsed_ms / K

@@ -113,14 +113,18 @@ class Pool {
         const bool pin = !(pin_env && pin_env[0] == '0') && !list.empty() && t <= (int)list.size();
         int offset = 0;
         if (const char *lr = getenv("LOCAL_RANK")) offset = atoi(lr) * t;      // local ranks take disjoint slices
+        // gen_ survives configure(): a new worker starts at the current generation, so that it answers only regions issued
+        // after it exists.  A worker starting below it would run a stale region and decrement pending_ twice, and
+        // parallel_for could return while another worker is still inside fn.  Read under api_, the only lock gen_ changes under.
+        const uint64_t start = gen_;
         for (int i = 1; i < t; i++) {
             const int cpu = pin ? list[(size_t)(offset + i) % list.size()] : -1;
-            workers_.emplace_back([this, cpu, list] {
+            workers_.emplace_back([this, cpu, list, start] {
                 cpu_set_t set; CPU_ZERO(&set);
                 if (cpu >= 0) CPU_SET(cpu, &set);
                 else for (int c : list) CPU_SET(c, &set);
                 if (cpu >= 0 || !cpus_.empty()) sched_setaffinity(0, sizeof set, &set);
-                uint64_t seen = 0;
+                uint64_t seen = start;
                 for (;;) {
                     {
                         std::unique_lock<std::mutex> lk(m_);

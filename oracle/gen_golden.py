@@ -10,7 +10,8 @@ Outputs
   tests/golden/trace_<inst>_<policy>.npz  step-by-step traces of the reference env:
         actions[T], mask[T+1, J+1] (row 0 = after reset), obs[T+1, J, 7] float64,
         reward[T] float64, done[T], t[T+1], nb_legal[T+1], nb_machine_legal[T+1],
-        plus the integer state arrays after every step
+        plus the integer state arrays after every step, stored in the lossless compact
+        form of compact_trace() (tests/helpers.py load_trace() reads both forms)
   tests/golden/known_answers.json       steps / makespan / sum(reward) of whole episodes under the
                                         deterministic "lowest/highest legal index" policies
   tests/golden/cr_factor_makespans.json CriticalRatio(due_date_factor=1.0 / 2.25 / 4.0), np.random.seed(0)
@@ -128,6 +129,23 @@ def record_trace(JssEnv, inst, policy, seed, max_steps=None):
     return arrays
 
 
+DELTA_CODED = ("t", "todo", "tufco", "tuam", "idle_last", "total_idle", "total_perform", "needed", "obs_index")
+
+
+def compact_trace(arrays):
+    """Lossless smaller form of a trace, so that a whole ta80 episode stays a small fixture: obs as int16 indices
+    into its distinct float64 values, and the slowly changing per-step integer arrays as differences between
+    consecutive steps (wrapping in their own dtype, which the running sum in load_trace() undoes exactly)."""
+    out = dict(arrays)
+    values, index = np.unique(out.pop("obs"), return_inverse=True)
+    assert len(values) <= np.iinfo(np.int16).max + 1
+    out["obs_values"], out["obs_index"] = values, index.reshape(arrays["obs"].shape).astype(np.int16)
+    for k in DELTA_CODED:
+        out[k] = np.diff(out[k], axis=0, prepend=np.zeros_like(out[k][:1]))
+    out["delta"] = np.array(DELTA_CODED)
+    return out
+
+
 def main():
     os.makedirs(GOLD, exist_ok=True)
     JssEnv, dispatching = load_reference()
@@ -143,7 +161,7 @@ def main():
     for inst, policy, seed, *cap in plan:
         arrays = record_trace(JssEnv, inst, policy, seed, cap[0] if cap else None)
         fn = os.path.join(GOLD, f"trace_{inst}_{policy}{seed}.npz")
-        np.savez_compressed(fn, **arrays)
+        np.savez_compressed(fn, **compact_trace(arrays))
         print(f"{fn}: steps={len(arrays['actions'])} makespan={arrays['t'][-1]} "
               f"sum_reward={arrays['reward'].sum()!r} size={os.path.getsize(fn)}")
 

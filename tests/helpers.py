@@ -24,6 +24,10 @@ def load_trace(path):
     z = np.load(path)
     J, M = [int(x) for x in z["shape"]]
     tr = {k: z[k] for k in z.files}
+    if "obs_index" in tr:                       # compact form (oracle/gen_golden.py compact_trace)
+        for k in tr.pop("delta"):
+            tr[k] = np.cumsum(tr[k], axis=0, dtype=tr[k].dtype)
+        tr["obs"] = tr.pop("obs_values")[tr.pop("obs_index")]
     tr["mask"] = np.unpackbits(z["mask"], axis=1)[:, : J + 1].astype(bool)
     tr["blocked"] = np.unpackbits(z["blocked"], axis=1)[:, :J].astype(bool)
     tr["machine_legal"] = np.unpackbits(z["machine_legal"], axis=1)[:, :M].astype(bool)

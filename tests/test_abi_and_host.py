@@ -26,15 +26,25 @@ def test_header_symbols_exported_by_cuda_library():
     assert lib.jss_abi_version() == _native.JSS_ABI_VERSION
 
 
+_NO_DEVICE_WORKER = r"""
+import sys
+sys.path.insert(0, {root!r})
+from jssenv_b200 import JssVecEnv
+from jssenv_b200._native import NativeError
+try:
+    JssVecEnv(2, {{"instance_path": "ta01"}})
+except NativeError as e:
+    print("NativeError:", e)
+"""
+
+
 def test_no_cpu_fallback_without_gpu():
-    """On a box without a CUDA device, constructing an env must fail loudly."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from jssenv_b200 import JssVecEnv
-    from jssenv_b200._native import NativeError
-    with pytest.raises(NativeError, match="no CUDA device|no CPU fallback"):
-        JssVecEnv(2, {"instance_path": "ta01"})
+    """On a box without a CUDA device, constructing an env must fail loudly.  The devices are hidden from a fresh
+    interpreter, so that this also holds where a GPU is present."""
+    r = subprocess.run([sys.executable, "-c", _NO_DEVICE_WORKER.format(root=ROOT)], capture_output=True, text=True,
+                       timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stdout + r.stderr
+    assert re.search(r"^NativeError:.*(no CUDA device|no CPU fallback)", r.stdout, re.M), r.stdout + r.stderr
 
 
 def test_buffers_struct_matches_header():
@@ -124,6 +134,17 @@ def test_markstein_division_is_exact_for_all_bundled_divisors(tmp_path):
         args += [str(y), str(y)]
     r = subprocess.run([str(exe)] + args, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "0 mismatches" in r.stdout, r.stdout[-400:]
+
+
+def test_host_pool_regions_complete_after_reconfigure(tmp_path):
+    """The host worker pool finishes every chunk of a parallel region before returning, also right after
+    jss_host_configure() restarted its workers, as bench.py's e2e calibration does (tools/check_pool.cpp)."""
+    exe = tmp_path / "check_pool"
+    csrc = os.path.join(ROOT, "jssenv_b200", "csrc")
+    subprocess.check_call(["g++", "-O2", "-std=c++17", "-I", csrc, "-o", str(exe), os.path.join(ROOT, "tools", "check_pool.cpp"),
+                           os.path.join(csrc, "jss_host.cpp"), "-lpthread"])
+    r = subprocess.run([str(exe), "2000"], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 0 and " 0 early returns" in r.stdout, r.stdout + r.stderr
 
 
 def test_step_kernels_compile_as_warp_convergent_code():
