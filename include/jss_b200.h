@@ -44,7 +44,7 @@
 extern "C" {
 #endif
 
-#define JSS_ABI_VERSION 2
+#define JSS_ABI_VERSION 3
 
 /* limits of the one-warp-per-env kernels */
 #define JSS_MAX_JOBS 256
@@ -160,6 +160,36 @@ int jss_get_buffers(jss_t *h, jss_buffers *out);
 /* derived per-instance scalars (jss_env.py:86-89): out[0]=max_time_op,
  * out[1]=max_time_jobs, out[2]=sum_op */
 int jss_instance_scalars(jss_t *h, int inst, int64_t out[3]);
+
+/* --- generator mode: a fresh random instance per env and episode ------------------------------------------
+ * Instance k of global env g (env_id_base + i) under instance seed s, for shape J x M and durations in
+ * [dmin, dmax], is a pure function of those values, computed with the same integer code on host and device
+ * (jssenv_b200/csrc/jss_gen.h):
+ *   h(c)            = jss_hash3(s ^ 0x6A09E667F3BCC909, g, c)     (the policy RNG uses jss_hash3(seed, g, step))
+ *   c(j, i, w)      = (k << 20) | (((j * M + i) << 1) | w)
+ *   duration[j][i]  = dmin + pick(h(c(j, i, 0)), dmax - dmin + 1)
+ *   machine[j]      = Fisher-Yates shuffle of 0..M-1 (Taillard): from the identity, for i = 0 .. M-2,
+ *                     r = i + pick(h(c(j, i, 1)), M - i), swap positions i and r;
+ *   pick(x, n)      = (x * n) >> 32 (64-bit product), jss_hash3 as in jssenv_b200/csrc/jss_rng.h.
+ * k counts the resets of the env: 0 at the reset jss_assign_generated performs, +1 at every later reset, explicit
+ * (jss_reset, masked or not) or automatic.  The stream does not depend on sharding; a second handle with the same
+ * seed replays it.  Limits: 2 <= M <= 32, 1 <= J <= 128, 1 <= dmin <= dmax <= 2047; all envs share one shape.
+ * In this mode jss_import_state, jss_step_export, jss_instance_scalars and the packed / hybrid host steps return
+ * JSS_ERR_UNSUPPORTED; everything else works as for loaded instances. */
+
+/* Takes the place of jss_load_instances + jss_assign on a fresh handle: allocates per-env instance tables,
+ * draws instance 0 of every env on the device and resets.  JSS_ERR_STATE after either of the two,
+ * JSS_ERR_UNSUPPORTED with JSS_CREATE_HOST_MIRROR. */
+int jss_assign_generated(jss_t *h, int jobs, int machines, int dur_min, int dur_max, uint64_t inst_seed);
+
+/* Each env's current instance: machine_dev / duration_dev int32 [N][J][M], index_dev int32 [N] (its k).
+ * Device pointers, any may be NULL; enqueued on `stream`. */
+int jss_get_env_instances(jss_t *h, int32_t *machine_dev, int32_t *duration_dev, int32_t *index_dev, void *stream);
+
+/* Host restatement of the generator (no device needed): instance `index` of env `env_id` into
+ * machine_host / duration_host int32 [J][M]. */
+int jss_generate_instance(int jobs, int machines, int dur_min, int dur_max, uint64_t inst_seed, uint64_t env_id,
+                          uint64_t index, int32_t *machine_host, int32_t *duration_host);
 
 /* --- hot path ------------------------------------------------------------ */
 

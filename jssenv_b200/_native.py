@@ -13,7 +13,7 @@ import numpy as np
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("JSS_B200_LIB") or os.path.join(_PKG_DIR, "libjss_b200.so")   # override: kernel-variant experiments only
 
-JSS_ABI_VERSION = 2
+JSS_ABI_VERSION = 3
 ACTION_SKIP, ACTION_ADVANCE = -1, -2
 CREATE_AUTO_RESET, CREATE_RECORD_SOLUTION, CREATE_HOST_MIRROR = 1, 2, 4
 FLAG_DONE, FLAG_ERROR, FLAG_NOOP_LEGAL = 1, 2, 4
@@ -29,6 +29,7 @@ EXPORTED_SYMBOLS = (
     "jss_step_host", "jss_host_step_begin", "jss_host_wait", "jss_step_sample", "jss_stats", "jss_export_state", "jss_import_state", "jss_host_masked_random",
     "jss_launch_count", "jss_set_cr_due_date_factor", "jss_host_step_begin_packed", "jss_host_wire_stride",
     "jss_host_expand_obs", "jss_host_configure", "jss_host_threads", "jss_host_set_simd", "jss_rollout_traj", "jss_step_export", "jss_host_step_begin_hybrid", "jss_host_expand_obs_range",
+    "jss_assign_generated", "jss_get_env_instances", "jss_generate_instance",
 )
 
 
@@ -97,9 +98,13 @@ def _declare(L):
     L.jss_set_cr_due_date_factor.restype = c_int
     L.jss_launch_count.argtypes = [c_void_p]
     L.jss_launch_count.restype = c_int64
+    L.jss_assign_generated.argtypes = [c_void_p, c_int, c_int, c_int, c_int, c_uint64]
+    L.jss_get_env_instances.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
+    L.jss_generate_instance.argtypes = [c_int, c_int, c_int, c_int, c_uint64, c_uint64, c_uint64, c_void_p, c_void_p]
     for name in ("jss_create", "jss_load_instances", "jss_assign", "jss_get_buffers", "jss_instance_scalars",
                  "jss_reset", "jss_step", "jss_policy", "jss_rollout", "jss_step_host", "jss_host_step_begin", "jss_host_wait", "jss_step_sample", "jss_stats",
-                 "jss_export_state", "jss_import_state", "jss_host_masked_random"):
+                 "jss_export_state", "jss_import_state", "jss_host_masked_random", "jss_assign_generated",
+                 "jss_get_env_instances", "jss_generate_instance"):
         getattr(L, name).restype = c_int
     return L
 

@@ -76,6 +76,10 @@ struct jss_handle {
     unsigned long long *d_stats = nullptr;
 
     JssParams p{};
+    // generator mode (jss_assign_generated): per-env instance tables, regenerated on the device at every reset
+    bool gen = false;
+    JssGenParams g{};
+    int gen_grid[24] = {0};                        // resident-CTA grids of the generator-mode kernel variants (filled lazily)
     JssSmemLayout sl_env{}, sl_step{}, sl_step_rem{};   // shared-memory layouts of the generic / step kernels (step: without / with the suffix-sum table)
     int class_tile_begin[4] = {0, 0, 0, 0}, class_tile_end[4] = {0, 0, 0, 0};  // KJ = 1, 2, 4, 8
     int step_grid[24] = {0};
@@ -258,7 +262,85 @@ int launch_class(jss_t *h, const JssLaunch &a, const JssSmemLayout &sl, cudaStre
     }
 }
 
+// ---- generator mode -------------------------------------------------------------------------------
+template <typename Kern>
+int gen_grid_for(jss_t *h, Kern kern, int slot, int threads, size_t smem) {
+    int &grid = h->gen_grid[slot];
+    if (grid == 0) {
+        if (smem > 48 * 1024)
+            JSS_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int per_sm = 0;
+        JSS_CUDA(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
+        if (per_sm < 1) return fail(h, JSS_ERR_CUDA, "generator-mode kernel does not fit on an SM (smem %zu B)", smem);
+        grid = h->sm_count * per_sm;
+    }
+    return JSS_OK;
+}
+
+template <int KJ, int SAMPLE>
+int launch_gen_step(jss_t *h, const JssLaunch &a_in, cudaStream_t st) {
+    JssLaunch a = a_in;
+    fill_uni(h->descs[0], a.uni);                        // the batch geometry (every env has the same shape)
+    JssGenStepArgs ga;
+    ga.sl = h->sl_step;                                  // no CTA-shared tables: the warp regions start at 0
+    ga.sl.off_warp0 = 0;
+    ga.g = h->g;
+    ga.g.off_gen = ga.sl.warp_stride;
+    ga.sl.warp_stride += (int32_t)sizeof(SmInst) + 2 * ga.g.tbl_bytes;
+    const size_t smem = (size_t)JSS_GEN_STEP_WARPS * ga.sl.warp_stride;
+    auto kern = jss_gen_step_kernel<KJ, SAMPLE>;
+    int rc = gen_grid_for(h, kern, class_of(KJ) * 4 + SAMPLE, JSS_GEN_STEP_WARPS * 32, smem);
+    if (rc) return rc;
+    const int grid = std::min(h->gen_grid[class_of(KJ) * 4 + SAMPLE], (h->n_envs + JSS_GEN_STEP_WARPS - 1) / JSS_GEN_STEP_WARPS);
+    if (h->use_pdl) JSS_CUDA(h, JSS_LAUNCH_PDL(kern, grid, JSS_GEN_STEP_WARPS * 32, smem, st, h->p, a, ga));
+    else JSS_LAUNCH(kern, grid, JSS_GEN_STEP_WARPS * 32, smem, st, h->p, a, ga);
+    JSS_CUDA(h, cudaGetLastError());
+    h->launches += 1;
+    return JSS_OK;
+}
+
+template <int KJ, int MODE>
+int launch_gen_env(jss_t *h, const JssLaunch &a_in, cudaStream_t st) {
+    JssLaunch a = a_in;
+    a.tile_begin = 0;
+    a.tile_end = (h->n_envs + JSS_WARPS_PER_CTA - 1) / JSS_WARPS_PER_CTA;
+    JssGenParams g = h->g;
+    g.warp_stride = (int32_t)sizeof(SmInst) + h->sl_env.scratch_words * 4;
+    const size_t smem = (size_t)JSS_WARPS_PER_CTA * g.warp_stride;
+    auto kern = jss_gen_env_kernel<KJ, MODE>;
+    const int slot = 12 + class_of(KJ) * 4 + (MODE == JSS_MODE_RESET ? 0 : MODE == JSS_MODE_ROLLOUT ? 1 : 2);
+    int rc = gen_grid_for(h, kern, slot, JSS_WARPS_PER_CTA * 32, smem);
+    if (rc) return rc;
+    // policy launches: latency-bound, one CTA per tile (as launch_variant)
+    const int grid = (MODE == JSS_MODE_POLICY) ? a.tile_end : std::min(a.tile_end, h->gen_grid[slot]);
+    JSS_LAUNCH(kern, grid, JSS_WARPS_PER_CTA * 32, smem, st, h->p, a, g);
+    JSS_CUDA(h, cudaGetLastError());
+    h->launches += 1;
+    return JSS_OK;
+}
+
+template <int KJ>
+int launch_gen_class(jss_t *h, const JssLaunch &a, cudaStream_t st) {
+    if (a.mode == JSS_MODE_STEP) {
+        const int sample = a.actions_out == nullptr ? 0 : (a.rule == JSS_RULE_RANDOM ? 1 : 2);
+        if (sample == 0) return launch_gen_step<KJ, 0>(h, a, st);
+        if (sample == 1) return launch_gen_step<KJ, 1>(h, a, st);
+        return launch_gen_step<KJ, 2>(h, a, st);
+    }
+    if (a.mode == JSS_MODE_POLICY) return launch_gen_env<KJ, JSS_MODE_POLICY>(h, a, st);
+    if (a.mode == JSS_MODE_ROLLOUT) return launch_gen_env<KJ, JSS_MODE_ROLLOUT>(h, a, st);
+    return launch_gen_env<KJ, JSS_MODE_RESET>(h, a, st);   // reset / export
+}
+
+int launch_gen(jss_t *h, const JssLaunch &a, cudaStream_t st) {
+    const int kj = kj_of(h->g.J);
+    if (kj == 1) return launch_gen_class<1>(h, a, st);
+    if (kj == 2) return launch_gen_class<2>(h, a, st);
+    return launch_gen_class<4>(h, a, st);
+}
+
 int launch_all(jss_t *h, JssLaunch a, bool want_rem, cudaStream_t st) {
+    if (h->gen) return launch_gen(h, a, st);
     if (a.mode == JSS_MODE_STEP && !a.export_after) return launch_step(h, a, st);   // one launch, whatever the mix of lane classes
     (void)want_rem;
     const JssSmemLayout &sl = h->sl_env;
@@ -371,39 +453,29 @@ int jss_load_instances(jss_t *h, int n_inst, const int32_t *jobs, const int32_t 
         ops.resize(ops.size() + round_up(J * M, 8), 0);
         len.resize(len.size() + round_up(J, 4), 0);
         rem.resize(rem.size() + round_up(J * (M + 1), 8), 0);
-        for (int j = 0; j < J; j++) {
-            int64_t total = 0;
-            for (int i = 0; i < M; i++) {
-                const int m = mm[j * M + i], t = dd[j * M + i];
-                if (m < 0 || m >= M) return fail(h, JSS_ERR_INVALID, "instance %d: machine %d out of range", k, m);
-                // Zero-length ops are rejected: the reference itself cannot finish such an episode -- an allocated op of
-                // duration 0 never satisfies `was_left_time > 0` (jss_env.py:529), so the job never advances to its
-                // next op and is re-legalised on the same machine at the same instant (jss_env.py:616-634).
-                if (t < 1 || t > JSS_MAX_DURATION)
-                    return fail(h, JSS_ERR_UNSUPPORTED, "instance %d: duration %d outside [1, %d]", k, t,
-                                JSS_MAX_DURATION);
-                ops[d.ops_off + j * M + i] = (uint16_t)((m << JSS_OP_SHIFT) | t);
-                total += t;
-                hi.max_time_op = std::max<int64_t>(hi.max_time_op, t);  // jss_env.py:86
-            }
-            len[d.len_off + j] = (int32_t)total;                        // jss_env.py:87
-            hi.len[j] = (int32_t)total;
-            hi.sum_op += total;                                         // jss_env.py:88
-            hi.max_time_jobs = std::max(hi.max_time_jobs, total);       // jss_env.py:89
-            int64_t suffix = 0;
-            rem[d.rem_off + j * (M + 1) + M] = 0;
-            for (int i = M - 1; i >= 0; i--) {
-                suffix += dd[j * M + i];
-                rem[d.rem_off + j * (M + 1) + i] = (uint16_t)suffix;    // <= 32 * 2047 < 65536
-            }
+        for (int q = 0; q < J * M; q++) {
+            const int m = mm[q], t = dd[q];
+            if (m < 0 || m >= M) return fail(h, JSS_ERR_INVALID, "instance %d: machine %d out of range", k, m);
+            // Zero-length ops are rejected: the reference itself cannot finish such an episode -- an allocated op of
+            // duration 0 never satisfies `was_left_time > 0` (jss_env.py:529), so the job never advances to its
+            // next op and is re-legalised on the same machine at the same instant (jss_env.py:616-634).
+            if (t < 1 || t > JSS_MAX_DURATION)
+                return fail(h, JSS_ERR_UNSUPPORTED, "instance %d: duration %d outside [1, %d]", k, t, JSS_MAX_DURATION);
         }
-        d.max_time_op = (int32_t)hi.max_time_op;
-        d.max_time_jobs = (int32_t)hi.max_time_jobs;
-        d.sum_op = (int32_t)hi.sum_op;
-        d.r_mto = 1.0f / (float)d.max_time_op;
-        d.r_mtj = 1.0f / (float)d.max_time_jobs;
-        d.r_sop = 1.0f / (float)d.sum_op;
-        d.r_M = 1.0f / (float)d.M;
+        for (int j = 0; j < J; j++) {
+            // tables + scalars of the row: the same code the device generator runs (jss_gen.h)
+            int32_t mx = 0;
+            const int32_t total = jss_pack_job_row(mm + j * M, dd + j * M, M, &ops[d.ops_off + j * M],
+                                                   &rem[d.rem_off + j * (M + 1)], &mx);
+            len[d.len_off + j] = total;                                 // jss_env.py:87
+            hi.len[j] = total;
+            hi.max_time_op = std::max<int64_t>(hi.max_time_op, mx);    // jss_env.py:86
+            hi.sum_op += total;                                         // jss_env.py:88
+            hi.max_time_jobs = std::max<int64_t>(hi.max_time_jobs, total);   // jss_env.py:89
+        }
+        const int32_t ops_off = d.ops_off, len_off = d.len_off, rem_off = d.rem_off;
+        d = jss_inst_desc(J, M, (int32_t)hi.max_time_op, (int32_t)hi.max_time_jobs, (int32_t)hi.sum_op);
+        d.ops_off = ops_off; d.len_off = len_off; d.rem_off = rem_off;
         h->insts[k] = hi;
         h->descs[k] = d;
     }
@@ -421,6 +493,8 @@ int jss_load_instances(jss_t *h, int n_inst, const int32_t *jobs, const int32_t 
 }
 
 int jss_instance_scalars(jss_t *h, int inst, int64_t out[3]) {
+    if (h && h->gen)
+        return fail(h, JSS_ERR_UNSUPPORTED, "jss_instance_scalars: generator mode has no instance list (see jss_get_env_instances)");
     if (!h || !out || !h->loaded || inst < 0 || inst >= (int)h->insts.size())
         return fail(h, JSS_ERR_INVALID, "jss_instance_scalars: bad arguments");
     out[0] = h->insts[inst].max_time_op;
@@ -429,10 +503,12 @@ int jss_instance_scalars(jss_t *h, int inst, int64_t out[3]) {
     return JSS_OK;
 }
 
-int jss_assign(jss_t *h, const int32_t *env_to_inst) {
-    if (!h || !env_to_inst) return fail(h, JSS_ERR_INVALID, "jss_assign: bad arguments");
-    if (!h->loaded) return fail(h, JSS_ERR_STATE, "jss_load_instances must be called first");
-    if (h->assigned) return fail(h, JSS_ERR_STATE, "envs already assigned");
+}  // extern "C"
+
+namespace {
+// grouping, shared-memory layouts and every per-env buffer of a batch whose instances are loaded (jss_assign), or
+// whose shape is (jss_assign_generated); ends with the first reset
+int assign_impl(jss_t *h, const int32_t *env_to_inst) {
     JSS_CUDA(h, cudaSetDevice(h->device));
     const int N = h->n_envs, n_inst = (int)h->insts.size();
     int jmax = 0, mmax = 0, ops_max = 0, rem_max = 0;
@@ -630,6 +706,93 @@ int jss_assign(jss_t *h, const int32_t *env_to_inst) {
     // a fresh batch starts reset, like a freshly constructed + reset reference env
     return jss_reset(h, nullptr, nullptr);
 }
+}  // namespace
+
+extern "C" {
+
+int jss_assign(jss_t *h, const int32_t *env_to_inst) {
+    if (!h || !env_to_inst) return fail(h, JSS_ERR_INVALID, "jss_assign: bad arguments");
+    if (!h->loaded) return fail(h, JSS_ERR_STATE, "jss_load_instances must be called first");
+    if (h->assigned) return fail(h, JSS_ERR_STATE, "envs already assigned");
+    return assign_impl(h, env_to_inst);
+}
+
+namespace {
+int check_gen_shape(jss_t *h, int jobs, int machines, int dur_min, int dur_max, const char *what) {
+    if (jobs < 1 || machines < 2 || dur_min > dur_max)
+        return fail(h, JSS_ERR_INVALID, "%s: need jobs >= 1, machines >= 2 and dur_min <= dur_max (got %dx%d, [%d, %d])",
+                    what, jobs, machines, dur_min, dur_max);
+    if (jobs > JSS_GEN_MAX_JOBS || machines > JSS_MAX_MACHINES || dur_min < 1 || dur_max > JSS_MAX_DURATION)
+        return fail(h, JSS_ERR_UNSUPPORTED, "%s: %dx%d with durations [%d, %d] exceeds the generator limits (%dx%d, [1, %d])",
+                    what, jobs, machines, dur_min, dur_max, JSS_GEN_MAX_JOBS, JSS_MAX_MACHINES, JSS_MAX_DURATION);
+    return JSS_OK;
+}
+}  // namespace
+
+int jss_assign_generated(jss_t *h, int jobs, int machines, int dur_min, int dur_max, uint64_t inst_seed) {
+    if (!h) return JSS_ERR_INVALID;
+    if (h->loaded || h->assigned)
+        return fail(h, JSS_ERR_STATE, "jss_assign_generated: takes the place of jss_load_instances + jss_assign on a fresh handle");
+    int rc = check_gen_shape(h, jobs, machines, dur_min, dur_max, "jss_assign_generated");
+    if (rc) return rc;
+    if (h->create_flags & JSS_CREATE_HOST_MIRROR)
+        return fail(h, JSS_ERR_UNSUPPORTED, "jss_assign_generated: JSS_CREATE_HOST_MIRROR is not available in generator mode");
+    JSS_CUDA(h, cudaSetDevice(h->device));
+    // the shape as the one "instance" of a uniform batch: state geometry, identity order and buffers come from it
+    const int J = jobs, M = machines, N = h->n_envs;
+    h->insts.assign(1, HostInst{J, M, 0, 0, 0, std::vector<int32_t>((size_t)J)});
+    JssInstDesc d{};
+    d.J = J; d.M = M;
+    h->descs.assign(1, d);
+    JssGenParams &g = h->g;
+    g.J = J; g.M = M; g.dmin = dur_min; g.dmax = dur_max; g.seed = inst_seed;
+    g.ops_bytes = 2 * round_up(J * M, 8);
+    g.tbl_bytes = JSS_GEN_HDR_BYTES + g.ops_bytes + 4 * round_up(J, 4);
+    g.rem_elems = round_up(J * (M + 1), 8);
+    g.n_envs = N;
+    if ((rc = dev_alloc(h, &g.tables, (size_t)N * g.tbl_bytes))) return rc;
+    if ((rc = dev_alloc(h, &g.rem, (size_t)N * g.rem_elems))) return rc;
+    if ((rc = dev_alloc(h, &g.index, (size_t)N, false))) return rc;
+    JSS_CUDA(h, cudaMemset(g.index, 0xff, (size_t)N * 4));   // -1: the first reset draws instance 0
+    h->gen = true;
+    h->loaded = true;
+    std::vector<int32_t> e2i((size_t)N, 0);
+    return assign_impl(h, e2i.data());
+}
+
+int jss_get_env_instances(jss_t *h, int32_t *machine_dev, int32_t *duration_dev, int32_t *index_dev, void *stream) {
+    int rc = check_ready(h);
+    if (rc) return rc;
+    if (!h->gen) return fail(h, JSS_ERR_STATE, "jss_get_env_instances: the handle is not in generator mode");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (machine_dev || duration_dev) {
+        const size_t total = (size_t)h->n_envs * h->g.J * h->g.M;
+        const int blocks = (int)std::min<size_t>((total + 255) / 256, (size_t)h->sm_count * 8);
+        JSS_LAUNCH(jss_gen_unpack_kernel, blocks, 256, 0, st, h->g, machine_dev, duration_dev);
+        JSS_CUDA(h, cudaGetLastError());
+        h->launches += 1;
+    }
+    if (index_dev)
+        JSS_CUDA(h, cudaMemcpyAsync(index_dev, h->g.index, (size_t)h->n_envs * 4, cudaMemcpyDeviceToDevice, st));
+    return JSS_OK;
+}
+
+int jss_generate_instance(int jobs, int machines, int dur_min, int dur_max, uint64_t inst_seed, uint64_t env_id,
+                          uint64_t index, int32_t *machine_host, int32_t *duration_host) {
+    if (!machine_host || !duration_host) return JSS_ERR_INVALID;
+    int rc = check_gen_shape(nullptr, jobs, machines, dur_min, dur_max, "jss_generate_instance");
+    if (rc) return rc;
+    uint8_t mach[JSS_MAX_MACHINES];
+    int32_t dur[JSS_MAX_MACHINES];
+    for (int j = 0; j < jobs; j++) {
+        jss_gen_row(inst_seed, env_id, index, j, machines, dur_min, dur_max, mach, dur);
+        for (int i = 0; i < machines; i++) {
+            machine_host[j * machines + i] = mach[i];
+            duration_host[j * machines + i] = dur[i];
+        }
+    }
+    return JSS_OK;
+}
 
 int jss_get_buffers(jss_t *h, jss_buffers *out) {
     if (!h || !out) return JSS_ERR_INVALID;
@@ -675,6 +838,7 @@ int jss_step_export(jss_t *h, const int32_t *actions_dev, void *stream) {
     int rc = check_ready(h);
     if (rc) return rc;
     if (!actions_dev) return fail(h, JSS_ERR_INVALID, "jss_step_export: actions_dev is NULL");
+    if (h->gen) return fail(h, JSS_ERR_UNSUPPORTED, "jss_step_export: not available in generator mode");
     JssLaunch a{};
     a.mode = JSS_MODE_STEP;
     a.actions = actions_dev;
@@ -769,6 +933,8 @@ int host_step_begin_impl(jss_t *h, const int32_t *actions_host, uint8_t *mask_ho
     int rc = check_ready(h);
     if (rc) return rc;
     if (!actions_host) return fail(h, JSS_ERR_INVALID, "jss_host_step_begin: actions_host is NULL");
+    if (wire_host && h->gen)   // the host expansion holds per-instance divisors
+        return fail(h, JSS_ERR_UNSUPPORTED, "packed / hybrid host steps are not available in generator mode");
     const JssParams &p = h->p;
     const size_t N = (size_t)p.n_envs;
     const size_t n_fp32 = obs_host ? (n_dma < 0 ? N : std::min<size_t>((size_t)n_dma, N)) : 0;     // envs [0, n_fp32): fp32 by DMA
@@ -886,6 +1052,7 @@ int jss_host_expand_obs_range(jss_t *h, const uint8_t *wire_host, const int32_t 
     if (!h || !h->assigned) return fail(h, JSS_ERR_STATE, "jss_host_expand_obs: jss_assign must be called first");
     if (!wire_host || !scalars_host || !obs_host || env_begin < 0 || env_end > h->n_envs || env_begin > env_end)
         return fail(h, JSS_ERR_INVALID, "jss_host_expand_obs: bad arguments");
+    if (h->gen) return fail(h, JSS_ERR_UNSUPPORTED, "jss_host_expand_obs: not available in generator mode");
     std::vector<JssHostInst> hi(h->insts.size());
     for (size_t k = 0; k < h->insts.size(); k++)
         hi[k] = JssHostInst{h->insts[k].J, h->insts[k].M, h->insts[k].max_time_op, h->insts[k].max_time_jobs,
@@ -982,6 +1149,8 @@ int jss_export_state(jss_t *h, void *stream) {
 int jss_import_state(jss_t *h, const uint8_t *env_mask_dev, void *stream) {
     int rc = check_ready(h);
     if (rc) return rc;
+    if (h->gen)   // a restored state would not match the instance the env has drawn since
+        return fail(h, JSS_ERR_UNSUPPORTED, "jss_import_state: not available in generator mode");
     JssLaunch a{};
     a.mode = JSS_MODE_IMPORT;
     a.env_mask = env_mask_dev;

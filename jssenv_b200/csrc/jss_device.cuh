@@ -27,6 +27,7 @@
 #include <string.h>
 
 #include "../../include/jss_b200.h"
+#include "jss_gen.h"
 #include "jss_rng.h"
 #include "jss_types.h"
 
@@ -185,6 +186,7 @@ JSS_DEV void jss_mbar_wait(jss_saddr_t mbar, uint32_t phase) {
     } while (!ok);
 }
 JSS_DEV void jss_fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+JSS_DEV void jss_fence_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 JSS_DEV void jss_bulk_store(void *gmem_dst, jss_saddr_t smem_src, uint32_t bytes) {   // joins the open bulk group
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
                  ::"l"(gmem_dst), "r"(smem_src), "r"(bytes) : "memory");
@@ -199,6 +201,14 @@ JSS_DEV void jss_bulk_commit() {
 }
 JSS_DEV void jss_bulk_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 JSS_DEV void jss_bulk_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+// several bulk loads completing on ONE mbarrier phase: one arrive announcing the total, then the copies
+JSS_DEV void jss_mbar_expect_tx(jss_saddr_t mbar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"(bytes) : "memory");
+}
+JSS_DEV void jss_bulk_copy(jss_saddr_t smem_dst, const void *gmem_src, uint32_t bytes, jss_saddr_t mbar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(smem_dst), "l"(gmem_src), "r"(bytes), "r"(mbar) : "memory");
+}
 #else   // host emulation (tests/emu): synchronous copies; the waits are warp rendezvous points
 typedef char *jss_saddr_t;
 JSS_DEV jss_saddr_t jss_saddr(const void *generic_ptr) { return (char *)generic_ptr; }
@@ -206,10 +216,13 @@ JSS_DEV void jss_mbar_init(jss_saddr_t) {}
 JSS_DEV void jss_bulk_load(jss_saddr_t smem_dst, const void *gmem_src, uint32_t bytes, jss_saddr_t) { memcpy(smem_dst, gmem_src, bytes); }
 JSS_DEV void jss_mbar_wait(jss_saddr_t, uint32_t) { __syncwarp(); }
 JSS_DEV void jss_fence_async_smem() {}
+JSS_DEV void jss_fence_async_global() {}
 JSS_DEV void jss_bulk_store(void *gmem_dst, jss_saddr_t smem_src, uint32_t bytes) { memcpy(gmem_dst, smem_src, bytes); }
 JSS_DEV void jss_bulk_commit() {}
 JSS_DEV void jss_bulk_store_wait_read() {}
 JSS_DEV void jss_bulk_store_wait_all() {}
+JSS_DEV void jss_mbar_expect_tx(jss_saddr_t, uint32_t) {}
+JSS_DEV void jss_bulk_copy(jss_saddr_t smem_dst, const void *gmem_src, uint32_t bytes, jss_saddr_t) { memcpy(smem_dst, gmem_src, bytes); }
 #endif
 
 // vector access to a lane's KJ-word slice
@@ -994,9 +1007,56 @@ JSS_DEV void env_emit_all(const JssParams &p, const InstView &iv, const EnvRegs<
     env_emit_scalars<KJ>(out, iv, s, env, lane, raw);
 }
 
-template <int KJ, int MODE>
+// ---- generator mode: draw instance k of an env (jss_gen.h) --------------------------------------------------
+// Lane l generates the rows of its KJ jobs; the three scalars are warp reductions, the reciprocals IEEE divisions, so the
+// desc and tables equal what jss_load_instances builds from the same arrays.  Writes the env's tables in HBM, the same
+// [desc][ops][len] unit into the warp's shared-memory table buffer `tb` (if given), and the warp's SmInst.
+template <int KJ>
+JSS_DEV void jss_gen_draw(const JssGenParams &g, uint64_t genv, int env, int k, int lane, char *tb, SmInst *si) {
+    const int J = g.J, M = g.M;
+    char *tg = g.tables + (size_t)env * g.tbl_bytes;
+    uint16_t *ops = reinterpret_cast<uint16_t *>(tg + JSS_GEN_HDR_BYTES);
+    int32_t *len = reinterpret_cast<int32_t *>(tg + JSS_GEN_HDR_BYTES + g.ops_bytes);
+    uint16_t *rem = g.rem + (size_t)env * g.rem_elems;
+    int32_t mto = 0, mtj = 0, sop = 0;
+#pragma unroll
+    for (int i = 0; i < KJ; i++) {
+        const int j = KJ * lane + i;
+        if (j < J) {
+            uint8_t mach[JSS_MAX_MACHINES];
+            int32_t dur[JSS_MAX_MACHINES];
+            jss_gen_row(g.seed, genv, (uint64_t)k, j, M, g.dmin, g.dmax, mach, dur);
+            int32_t mx = 0;
+            const int32_t l = jss_pack_job_row(mach, dur, M, ops + j * M, rem + j * (M + 1), &mx);
+            len[j] = l;
+            if (tb) {
+                uint16_t *so = reinterpret_cast<uint16_t *>(tb + JSS_GEN_HDR_BYTES) + j * M;
+                for (int q = 0; q < M; q++) so[q] = ops[j * M + q];
+                reinterpret_cast<int32_t *>(tb + JSS_GEN_HDR_BYTES + g.ops_bytes)[j] = l;
+            }
+            mto = max(mto, mx); mtj = max(mtj, l); sop += l;
+        }
+    }
+    mto = (int32_t)__reduce_max_sync(JSS_FULL, (unsigned)mto);
+    mtj = (int32_t)__reduce_max_sync(JSS_FULL, (unsigned)mtj);
+    sop = (int32_t)__reduce_add_sync(JSS_FULL, (unsigned)sop);
+    if (lane == 0) {
+        const JssInstDesc d = jss_inst_desc(J, M, mto, mtj, sop);
+        *reinterpret_cast<JssInstDesc *>(tg) = d;
+        if (tb) *reinterpret_cast<JssInstDesc *>(tb) = d;
+        jss_fill_sminst(d, si);
+        g.index[env] = k;
+    }
+    // the tables were written through the generic proxy; the step kernel reads them with bulk copies (async proxy)
+    jss_fence_async_global();
+    __syncwarp();
+}
+
+// GEN: generator mode (jss_gen_env_kernel): `iv` points at the env's own tables, iv.si at the warp's own SmInst, and every
+// reset -- explicit, or the auto-reset inside a rollout -- first draws the env's next instance.
+template <int KJ, int MODE, bool GEN = false>
 JSS_DEV void jss_process_env(const JssParams &p, const JssLaunch &a, const InstView &iv, int env, int lane,
-                             float *scratch) {
+                             float *scratch, const JssGenParams *g = nullptr) {
     EnvRegs<KJ> s;
     // MODE is a compile-time kernel variant (the hot step kernel carries no policy /
     // rollout / export code); JSS_MODE_RESET instantiates the rarely used rest
@@ -1004,6 +1064,7 @@ JSS_DEV void jss_process_env(const JssParams &p, const JssLaunch &a, const InstV
     int *hz = reinterpret_cast<int *>(scratch);
     if (mode == JSS_MODE_RESET) {
         if (a.env_mask && a.env_mask[env] == 0) return;
+        if (GEN) jss_gen_draw<KJ>(*g, p.env_id_base + (uint64_t)env, env, g->index[env] + 1, lane, nullptr, const_cast<SmInst *>(iv.si));
         env_reset_regs<KJ>(iv, s, lane);
         if (p.solution) {
             int32_t *sol = p.solution + (size_t)env * p.jobs_max * p.machines_max;
@@ -1065,6 +1126,8 @@ JSS_DEV void jss_process_env(const JssParams &p, const JssLaunch &a, const InstV
     for (int k = 0; k < a.n_steps; k++) {
         const uint32_t h = jss_hash3(a.seed, genv, a.step_index + (uint64_t)k);
         const int act = jss_uniform(env_select_action<KJ>(iv, s, lane, a.rule, a.coin_mode, h, a.cr_factor));
+        if (GEN && (s.flags & JSS_FLAG_DONE) && (p.create_flags & JSS_CREATE_AUTO_RESET))   // env_step resets it now
+            jss_gen_draw<KJ>(*g, genv, env, g->index[env] + 1, lane, nullptr, const_cast<SmInst *>(iv.si));
         int r = 0;
         const bool changed = env_step<KJ>(p, iv, s, env, lane, act, r, hz);
         s.flags = jss_uniform(s.flags);
@@ -1132,6 +1195,33 @@ jss_env_kernel(const JssParams p, const JssLaunch a, const JssSmemLayout sl) {
         if (warp < count)
             jss_process_env<KJ, MODE>(p, a, iv, p.uniform_inst >= 0 ? first + warp : jss_uniform(p.order[first + warp]),
                                       lane, scratch);
+    }
+}
+
+// Generator mode, everything but the step (reset, policy, rollout, export): uniform geometry and identity order like a
+// uniform batch, but each warp points its InstView at its own env's tables in HBM and keeps its own SmInst in shared
+// memory -- no CTA barrier.  Per warp: [SmInst][scratch], g.warp_stride bytes.
+template <int KJ, int MODE>
+__global__ void __launch_bounds__(JSS_WARPS_PER_CTA * 32, 1)
+jss_gen_env_kernel(const JssParams p, const JssLaunch a, const JssGenParams g) {
+    JSS_SMEM_DECL(jss_smem);
+    const int warp = jss_warp_index(), lane = threadIdx.x & 31;
+    char *wb = reinterpret_cast<char *>(jss_smem) + warp * g.warp_stride;
+    SmInst *si = reinterpret_cast<SmInst *>(wb);
+    float *scratch = reinterpret_cast<float *>(wb + sizeof(SmInst));
+    InstView iv;
+    iv.si = si; iv.staged = true; iv.Ju = g.J; iv.Mu = g.M;
+    for (int tile = a.tile_begin + (int)blockIdx.x; tile < a.tile_end; tile += (int)gridDim.x) {
+        const int env = tile * JSS_WARPS_PER_CTA + warp;
+        if (env >= p.n_envs) break;
+        const char *tg = g.tables + (size_t)env * g.tbl_bytes;
+        iv.ops = reinterpret_cast<const uint16_t *>(tg + JSS_GEN_HDR_BYTES);
+        iv.len = reinterpret_cast<const int32_t *>(tg + JSS_GEN_HDR_BYTES + g.ops_bytes);
+        iv.rem = g.rem + (size_t)env * g.rem_elems;
+        if (lane == 0) jss_fill_sminst(*reinterpret_cast<const JssInstDesc *>(tg), si);
+        __syncwarp();
+        jss_process_env<KJ, MODE, true>(p, a, iv, env, lane, scratch, &g);
+        __syncwarp();                                    // every lane is done with si before the next env refills it
     }
 }
 
@@ -1344,6 +1434,120 @@ jss_step_mixed_kernel(const JssParams p, const JssLaunch a, const JssSmemLayout 
     jss_step_tiles<2, SAMPLE, false>(p, a, sl, iv, c, w, warp, lane, r0.z, r0.w, 1, staged, phase);
     jss_step_tiles<1, SAMPLE, false>(p, a, sl, iv, c, w, warp, lane, r1.x, r1.y, 1, staged, phase);
     if (lane == 0) jss_bulk_store_wait_all();            // shared memory must outlive the bulk reads
+}
+
+// Generator mode (every env has its own instance): the structure of the uniform step kernel -- persistent CTAs, static
+// strided envs, the next env's state block prefetched by TMA -- plus, in the same bulk batch on the same mbarrier, that
+// env's [desc][ops][len] table unit into the other half of a double-buffered per-warp table buffer (the current env reads
+// its half for the whole step).  The suffix sums (only MWR / LWR / CR read them) are read through L1 from HBM.
+// A done env that auto-resets draws its next instance here, before env_step's reset path runs.
+// Per warp, behind the step region of jss_step_carve: [SmInst][table unit 0][table unit 1].
+#ifndef JSS_GEN_STEP_WARPS
+#define JSS_GEN_STEP_WARPS 4   // 4-warp CTAs: the double-buffered tables of 100x20 envs take 16 KB of shared memory per warp
+#endif
+struct JssGenStepArgs {      // shared-memory layout + generator-mode tables of the step kernel
+    JssSmemLayout sl;
+    JssGenParams g;
+};
+template <int KJ, int SAMPLE>
+__global__ void __launch_bounds__(JSS_GEN_STEP_WARPS * 32, KJ == 1 ? 2 * JSS_MIN_CTAS_SMALL : 2 * JSS_MIN_CTAS)
+jss_gen_step_kernel(const JssParams p, const JssLaunch a, const JssGenStepArgs ga) {
+    const JssSmemLayout &sl = ga.sl;
+    const JssGenParams &g = ga.g;
+    JSS_SMEM_DECL(jss_smem);
+    char *sm = reinterpret_cast<char *>(jss_smem);
+    const int warp = jss_warp_index(), lane = threadIdx.x & 31;
+    JssWarpSmem w;
+    jss_step_carve(sl, sm, warp, w);
+    char *wg = sm + sl.off_warp0 + warp * sl.warp_stride + g.off_gen;
+    SmInst *si = reinterpret_cast<SmInst *>(wg);
+    char *tb0 = wg + sizeof(SmInst);
+    const jss_saddr_t tb0_sa = w.mbar + (uint32_t)(g.off_gen + (int)sizeof(SmInst));
+    if (lane == 0) jss_mbar_init(w.mbar);
+    jss_pdl_launch_dependents();
+    __syncwarp();
+    jss_pdl_wait();
+    InstView iv;
+    iv.si = si; iv.staged = true; iv.Ju = g.J; iv.Mu = g.M;
+    const uint32_t blk16 = (uint32_t)a.uni.block_words >> 2, tbl_bytes = (uint32_t)g.tbl_bytes;
+    const int env_step_stride = (int)gridDim.x * JSS_GEN_STEP_WARPS;
+    uint32_t phase = 0, buf = 0;
+    int env_next = (int)blockIdx.x * JSS_GEN_STEP_WARPS + warp, act_next = 0;
+    if (env_next < p.n_envs) {
+        if (lane == 0) {
+            jss_mbar_expect_tx(w.mbar, blk16 * 16u + tbl_bytes);
+            jss_bulk_copy(w.state_sa, p.state + (size_t)env_next * blk16 * 4, blk16 * 16u, w.mbar);
+            jss_bulk_copy(tb0_sa, g.tables + (size_t)env_next * tbl_bytes, tbl_bytes, w.mbar);
+        }
+        act_next = a.actions[env_next];
+    }
+    while (env_next < p.n_envs) {
+        const int env = env_next, action = act_next;
+        char *tb = tb0 + buf * tbl_bytes;
+        jss_mbar_wait(w.mbar, phase);                    // this env's state block and tables have landed
+        phase ^= 1u;
+        iv.ops = reinterpret_cast<const uint16_t *>(tb + JSS_GEN_HDR_BYTES);
+        iv.len = reinterpret_cast<const int32_t *>(tb + JSS_GEN_HDR_BYTES + g.ops_bytes);
+        iv.rem = g.rem + (size_t)env * g.rem_elems;
+        if (lane == 0) jss_fill_sminst(*reinterpret_cast<const JssInstDesc *>(tb), si);
+        __syncwarp();
+        EnvRegs<KJ> s;
+        env_load_from<KJ>(p, iv, w.state_in, lane, s);
+        __syncwarp();                                    // every lane has read the state buffer
+        env_next = env + env_step_stride;
+        // the warp's generic-proxy accesses of the buffers the prefetch overwrites (the state buffer just read, the other
+        // table half, which the generator may have written two envs ago) must be ordered before its async-proxy writes:
+        // without this fence, 65 536-env runs of 100x20 saw torn tables after auto-resets (observations outside [0, 1])
+        jss_fence_async_smem();
+        __syncwarp();
+        if (env_next < p.n_envs) {                       // prefetch the next env's block + tables + action
+            if (lane == 0) {
+                jss_mbar_expect_tx(w.mbar, blk16 * 16u + tbl_bytes);
+                jss_bulk_copy(w.state_sa, p.state + (size_t)env_next * blk16 * 4, blk16 * 16u, w.mbar);
+                jss_bulk_copy(tb0_sa + (buf ^ 1u) * tbl_bytes, g.tables + (size_t)env_next * tbl_bytes, tbl_bytes, w.mbar);
+            }
+            act_next = a.actions[env_next];
+        }
+        s.flags = jss_uniform(s.flags);
+        if ((s.flags & JSS_FLAG_DONE) && action != JSS_ACTION_SKIP && (p.create_flags & JSS_CREATE_AUTO_RESET))
+            jss_gen_draw<KJ>(g, p.env_id_base + (uint64_t)env, env, g.index[env] + 1, lane, tb, si);
+        int raw = 0;
+        // the previous env's observation must have left the staging buffer (also aliased by hz)
+        if (lane == 0) jss_bulk_store_wait_read();
+        __syncwarp();
+        const uint32_t flags_in = s.flags;
+        const bool changed = env_step<KJ>(p, iv, s, env, lane, action, raw, reinterpret_cast<int *>(w.scratch));
+        s.flags = jss_uniform(s.flags);
+        if (SAMPLE) {
+            const uint32_t h = jss_hash_env(a.hash_key, p.env_id_base + (uint64_t)env);   // == jss_hash3(seed, genv, step_index)
+            const int nxt = env_select_action<KJ, SAMPLE == 1>(iv, s, lane, a.rule, a.coin_mode, h, a.cr_factor);
+            if (lane == 0) a.actions_out[env] = nxt;
+        }
+        if (changed) {
+            env_store_to<KJ>(p, iv, w.state_out, lane, s);
+            env_emit_all<KJ, true>(p, iv, s, env, lane, w.scratch, raw, w.scratch_sa,
+                                   p.state + (size_t)env * blk16 * 4, w.state_out_sa, blk16 * 16u);
+        } else if (s.flags != flags_in) {                // only the sticky error bit changed
+            if (lane == 0) {
+                p.state[(size_t)p.hdr_off16[env] * 4 + JSS_HDR_FLAGS] = (int32_t)s.flags;
+                reinterpret_cast<int4 *>(p.scalars)[env] =
+                    make_int4(0, 0, s.t, (int)((s.flags << 8) | (s.flags & JSS_FLAG_DONE)));
+            }
+        }
+        buf ^= 1u;
+    }
+    if (lane == 0) jss_bulk_store_wait_all();            // shared memory must outlive the bulk reads
+}
+
+// generator mode: every env's current instance as machine / duration arrays [N][J][M]
+__global__ void jss_gen_unpack_kernel(const JssGenParams g, int32_t *machine, int32_t *duration) {
+    const size_t jm = (size_t)g.J * g.M, total = (size_t)g.n_envs * jm;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t e = i / jm, q = i % jm;
+        const uint32_t op = reinterpret_cast<const uint16_t *>(g.tables + e * g.tbl_bytes + JSS_GEN_HDR_BYTES)[q];
+        if (machine) machine[i] = (int32_t)(op >> JSS_OP_SHIFT);
+        if (duration) duration[i] = (int32_t)(op & JSS_OP_DMASK);
+    }
 }
 
 // ---- SM-driven copy of small results into mapped pinned host memory -------------------------

@@ -115,6 +115,25 @@ struct JssLaunch {           // per-launch arguments
     SmInst uni;              // scalars of the single instance of a uniform batch (step kernel, UNI = true)
 };
 
+// Generator mode (jss_assign_generated): every env has its own instance tables in HBM, regenerated on the device at
+// each of its resets.  Per env, `tables + env * tbl_bytes` holds [JssInstDesc, padded to 64 B][ops u16][len i32] (the
+// unit the step kernel prefetches with one bulk copy), `rem + env * rem_elems` the suffix sums, `index[env]` the number
+// k of the instance it runs (-1 before the first reset).  The kernels of this mode take it as an extra parameter.
+#define JSS_GEN_HDR_BYTES 64
+struct JssGenParams {
+    int32_t J, M, dmin, dmax;
+    uint64_t seed;
+    char *tables;
+    uint16_t *rem;
+    int32_t *index;
+    int32_t tbl_bytes;      // 64 + ops_bytes + 4 * round_up(J, 4)
+    int32_t ops_bytes;      // 2 * round_up(J * M, 8)
+    int32_t rem_elems;      // round_up(J * (M + 1), 8)
+    int32_t n_envs;
+    int32_t warp_stride;    // bytes per warp region: step kernel [step-kernel region][SmInst][tables x 2], generic [SmInst][scratch]
+    int32_t off_gen;        // step kernel: offset of [SmInst][tables x 2] inside the warp region
+};
+
 #define JSS_MODE_RESET 0
 #define JSS_MODE_STEP 1
 #define JSS_MODE_ROLLOUT 2

@@ -95,3 +95,20 @@ def write_taillard(spec, path) -> str:
         for j in range(J):
             f.write(" ".join(f"{int(machine[j, i])} {int(duration[j, i])}" for i in range(M)) + "\n")
     return os.fspath(path)
+
+
+def generate_instance(jobs: int, machines: int, duration: Tuple[int, int], seed: int, env_id: int,
+                      index: int) -> Tuple[np.ndarray, np.ndarray]:
+    """Instance `index` of global env `env_id` in generator mode (``{"generator": ...}`` env configs), computed on the
+    host by the library's own generator (jss_generate_instance) -> (machine[J, M], duration[J, M]) int32."""
+    import ctypes
+    from . import _native
+    machine = np.empty((jobs, machines), np.int32)
+    dur = np.empty((jobs, machines), np.int32)
+    rc = _native.backend.library().jss_generate_instance(int(jobs), int(machines), int(duration[0]), int(duration[1]),
+                                                         int(seed), int(env_id), int(index),
+                                                         ctypes.c_void_p(machine.ctypes.data), ctypes.c_void_p(dur.ctypes.data))
+    if rc != 0:
+        msg = _native.backend.library().jss_last_error(None)
+        raise _native.NativeError(f"jss_generate_instance failed (rc={rc}): {msg.decode() if msg else ''}")
+    return machine, dur

@@ -41,12 +41,34 @@ class JssVecEnv:
         self.env_id_base = int(env_id_base)
         self.auto_reset = bool(auto_reset)
         self._step_index = 0
-        insts, env_to_inst = _instance_list(env_config)
-        self.instances = insts
         flags = ((N.CREATE_AUTO_RESET if auto_reset else 0) | (N.CREATE_RECORD_SOLUTION if record_solution else 0) |
                  (N.CREATE_HOST_MIRROR if host_mirror else 0))
         rc = self._L.jss_create(ctypes.byref(self._h), self.device_index, self.num_envs, flags, self.env_id_base)
         N.check(None, rc, "jss_create")
+        self.generator = None
+        if env_config is not None and "generator" in env_config:
+            self._assign_generated(env_config["generator"])
+        else:
+            self._assign_instances(env_config)
+        self._bind_buffers()
+
+    def _assign_generated(self, gen: Dict[str, Any]):
+        """Generator mode: a fresh random J x M instance per env and episode, drawn on the device (jss_assign_generated)."""
+        J, M = int(gen["jobs"]), int(gen["machines"])
+        dmin, dmax = (int(v) for v in gen.get("duration", (1, 99)))
+        seed = int(gen.get("seed", self.seed))
+        self.generator = {"jobs": J, "machines": M, "duration": (dmin, dmax), "seed": seed}
+        rc = self._L.jss_assign_generated(self._h, J, M, dmin, dmax, seed)   # also draws instance 0 and resets
+        N.check(self._h, rc, "jss_assign_generated")
+        self.instances = None
+        self.instance_scalars = None
+        self.env_to_instance = None
+        self.env_jobs = np.full(self.num_envs, J, np.int32)
+        self.env_machines = np.full(self.num_envs, M, np.int32)
+
+    def _assign_instances(self, env_config):
+        insts, env_to_inst = _instance_list(env_config)
+        self.instances = insts
         # instance tables (jss_env.py:72-95)
         jobs = np.array([m.shape[0] for m, _ in insts], np.int32)
         machines = np.array([m.shape[1] for m, _ in insts], np.int32)
@@ -71,6 +93,8 @@ class JssVecEnv:
             N.check(self._h, self._L.jss_instance_scalars(
                 self._h, k, sc[k].ctypes.data_as(ctypes.POINTER(ctypes.c_int64))), "jss_instance_scalars")
         self.instance_scalars = sc                           # max_time_op, max_time_jobs, sum_op
+
+    def _bind_buffers(self):
         b = N.JssBuffers()
         N.check(self._h, self._L.jss_get_buffers(self._h, ctypes.byref(b)), "jss_get_buffers")
         self._b = b
@@ -380,6 +404,21 @@ class JssVecEnv:
         rc = self._L.jss_stats(self._h, out.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), self._stream())
         N.check(self._h, rc, "jss_stats")
         return dict(zip(N.STATS_KEYS, (int(v) for v in out)))
+
+    def env_instances(self) -> Dict[str, Any]:
+        """Generator mode: every env's current instance as device tensors {"machine": (N, J, M), "duration": (N, J, M),
+        "index": (N,)} int32 -- index = how many resets the env has had since the first (the k of its instance)."""
+        import torch
+        if self.generator is None:
+            raise N.NativeError("env_instances() needs a generator-mode env ({'generator': ...} config)")
+        n, J, M = self.num_envs, self.jobs, self.machines
+        out = {"machine": torch.empty((n, J, M), dtype=torch.int32, device=self.device),
+               "duration": torch.empty((n, J, M), dtype=torch.int32, device=self.device),
+               "index": torch.empty((n,), dtype=torch.int32, device=self.device)}
+        rc = self._L.jss_get_env_instances(self._h, *(ctypes.c_void_p(out[k].data_ptr()) for k in ("machine", "duration", "index")),
+                                           self._stream())
+        N.check(self._h, rc, "jss_get_env_instances")
+        return out
 
     def export_state(self) -> Dict[str, Any]:
         """Canonical per-env integer state as device tensors (snapshot); see jss_b200.h."""
